@@ -54,6 +54,11 @@ WORKLOADS = {
     "cart512": ("cart", (8, 8, 8), "tooling: 512 hexes (compute-sanitizer runs)"),
 }
 CPU_SAMPLE = {"tet": (8, 8, 8), "cart": (20, 20, 20)}   # 3,072 tets / 8,000 hexes: 10-20 s of reference time
+# the value arrays one step assembles, in the order of the plan's output keys (PB_OUT_* in include/poreb200.h)
+STEP_OUTPUTS = ("flux", "bound_flux", "bound_pressure_cell", "bound_pressure_face", "vector_source",
+                "bound_pressure_vector_source", "stress", "bound_stress", "bound_displacement_cell",
+                "bound_displacement_face")
+DUMP_BYTES = 64 << 20
 
 
 def make_grid(kind, dims, seed=0):
@@ -376,6 +381,20 @@ def md_network_block(kind, dims, solve=True, newton=True):
     return out
 
 
+def dump_outputs(out_dir, outputs):
+    """Write each ``DeviceValues`` of ``outputs`` to ``out_dir/<name>.npy`` (float64), at most ``DUMP_BYTES`` in all: an
+    array longer than its share is cut to a sample at seeded positions, the same in every run on the same workload, so
+    that the files of two builds compare entry by entry.  The kernels add the contributions of the interaction regions
+    with atomics, so two runs of one build agree in all but the last bits, not bit for bit."""
+    os.makedirs(out_dir, exist_ok=True)
+    cap = (DUMP_BYTES - 4096) // (8 * len(outputs))          # 4 KB for the .npy headers
+    for name, vals in outputs.items():
+        v = vals.download()
+        if v.size > cap:
+            v = v[np.sort(np.random.default_rng(0).choice(v.size, cap, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), np.array(v, dtype=np.float64))
+
+
 def pinned_copy(a):
     """Page-locked copy of a host array (the e2e inputs are read by H2D copies at full PCIe rate)."""
     from porepy_b200 import _lib
@@ -414,7 +433,12 @@ def main():
     ap.add_argument("--no-krylov", action="store_true")
     ap.add_argument("--no-mech-solve", action="store_true", help="skip the block-Jacobi solve of the mechanics system")
     ap.add_argument("--no-md-network", action="store_true", help="skip the mixed-dimensional fracture-network extra (N = 1)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the ten matrices' value arrays of the last timed step (rank 0) to DIR/<name>.npy, "
+                         "float64, 64 MB in all (seeded samples of the larger arrays)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -530,6 +554,9 @@ def main():
     sz = plan.sizes()
     regions_all = allsum([float((shard.own_node.sum() if shard is not None else g.num_nodes))])[0]
     cells_all = allsum([float(nc)])[0]
+    # the last step's results stay in HBM, detached from the plan, and are written after the JSON line
+    last_outputs = ({name: plan.take(key) for key, name in enumerate(STEP_OUTPUTS)}
+                    if args.dump_outputs and rank == 0 else None)
     del plan
     if hasattr(g, "_b200_plan"):
         del g._b200_plan
@@ -836,6 +863,8 @@ def main():
         "spmv": spmv, "krylov": krylov, "md_network": md, "cpu_baseline": cpu,
     }
     emit(json.dumps(line))
+    if last_outputs is not None:
+        dump_outputs(args.dump_outputs, last_outputs)
     if dist is not None:
         dist.barrier()
         dist.destroy_process_group()

@@ -12,10 +12,10 @@ rm -rf "$here/_ref"
 mkdir -p "$here/_ref"
 cp -r "$src" "$here/_ref/porepy"
 find "$here/_ref" -name __pycache__ -type d -prune -exec rm -rf {} +
-# the reference's own unit tests of the path (collected where they lie by tools/run_reference_tests.py)
+# the reference's own unit tests of the path, in the same layout (collected there by tools/run_reference_tests.py)
 if [ -d "$(dirname "$(dirname "$src")")/tests/numerics/fv" ]; then
-  mkdir -p "$here/_ref_tests"
-  cp -r "$(dirname "$(dirname "$src")")/tests/numerics/fv" "$here/_ref_tests/fv"
-  find "$here/_ref_tests" -name __pycache__ -type d -prune -exec rm -rf {} +
+  mkdir -p "$here/_ref/tests/numerics"
+  cp -r "$(dirname "$(dirname "$src")")/tests/numerics/fv" "$here/_ref/tests/numerics/fv"
+  find "$here/_ref/tests" -name __pycache__ -type d -prune -exec rm -rf {} +
 fi
 du -sh "$here/_ref"

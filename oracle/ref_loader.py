@@ -18,6 +18,9 @@ from unittest.mock import MagicMock
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _CANDIDATES = ["/root/reference/src", os.path.join(_HERE, "_ref")]
 REF_SRC = next((p for p in _CANDIDATES if os.path.isdir(os.path.join(p, "porepy"))), _CANDIDATES[0])
+# the reference's own test suite: next to src/ in the reference tree, inside the copy under oracle/_ref
+REF_TESTS = next((p for p in (os.path.join(os.path.dirname(REF_SRC), "tests"), os.path.join(REF_SRC, "tests"))
+                  if os.path.isdir(p)), None)
 
 _STUBS = [
     "meshio", "gmsh", "shapely", "shapely.geometry", "shapely.speedups",

@@ -1,16 +1,13 @@
 """``porepy_b200.ad_functions`` against the reference's ``pp.ad.functions`` / ``AdArray.__pow__`` on random ``AdArray``s
-(value and Jacobian), incl. the tie rule of ``maximum`` and the zero-vector rule of ``l2_norm``.
-CPU: the scipy stand-in for the device sparse algebra (needs the reference: build container); GPU leg at the end of the suite."""
+(value and Jacobian), incl. the tie rule of ``maximum`` and the zero-vector rule of ``l2_norm``.  The reference's results
+are stored in tests/golden/ad_functions.npz (tools/make_ad_functions_golden.py).
+CPU: the scipy stand-in for the device sparse algebra; GPU leg at the end of the suite."""
 import os
-import sys
 
 import numpy as np
-import pytest
 import scipy.sparse as sps
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path.insert(0, os.path.join(ROOT, "tools"))
-from ref_loader import load_porepy, reference_available  # noqa: E402
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ad_functions.npz")
 
 
 def cases(n=24, m=40, seed=0):
@@ -26,51 +23,61 @@ def cases(n=24, m=40, seed=0):
     return dict(a=(a, jac()), b=(b, jac()), c=(c, jac()), pos=(pos, jac()))
 
 
-def run_checks(make, fn, to_host, pp):
-    """``make(val, jac)`` builds the device array; ``fn`` is porepy_b200.ad_functions."""
-    f = pp.ad.functions
-    A = pp.ad.AdArray
-    cs = cases()
-    ref = {k: A(v.copy(), j.copy()) for k, (v, j) in cs.items()}
-    dev = {k: make(v, j) for k, (v, j) in cs.items()}
+def reference_results():
+    """label -> (value, Jacobian or None) of the reference on ``cases()``."""
+    d = np.load(GOLDEN)
+    out = {}
+    for key in d.files:
+        if key.endswith("__val"):
+            j = key[:-5] + "__jac"
+            out[key[:-5]] = (d[key], sps.csr_matrix((d[j + "__data"], d[j + "__indices"], d[j + "__indptr"]),
+                                                    shape=tuple(d[j + "__shape"])) if j + "__data" in d.files else None)
+    return out
 
-    def same(r, g, what):
-        rv, rj = (r.val, r.jac) if isinstance(r, A) else (np.asarray(r), None)
+
+def run_checks(make, fn, to_host):
+    """``make(val, jac)`` builds the device array; ``fn`` is porepy_b200.ad_functions."""
+    ref = reference_results()
+    cs = cases()
+    dev = {k: make(v, j) for k, (v, j) in cs.items()}
+    checked = set()
+
+    def same(what, g):
+        rv, rj = ref[what]
         gv, gj = to_host(g)
         assert np.allclose(gv, rv, rtol=1e-13, atol=1e-13), what
         if rj is not None:
-            d = abs(sps.csr_matrix(rj) - sps.csr_matrix(gj))
-            assert (d.max() if d.nnz else 0.0) <= 1e-12 * max(abs(sps.csr_matrix(rj)).max(), 1.0), what
-    same(f.exp(ref["a"]), fn.exp(dev["a"]), "exp")
-    same(f.log(ref["pos"]), fn.log(dev["pos"]), "log")
-    same(f.abs(ref["a"]), fn.abs(dev["a"]), "abs")
-    same(f.sin(ref["a"]), fn.sin(dev["a"]), "sin")
-    same(f.cos(ref["a"]), fn.cos(dev["a"]), "cos")
-    same(f.tanh(ref["a"]), fn.tanh(dev["a"]), "tanh")
-    same(ref["pos"] ** 2.5, fn.power(dev["pos"], 2.5), "pow")
-    same(ref["pos"] ** 0.5, fn.sqrt(dev["pos"]), "sqrt")
-    same(f.heaviside(0.5, ref["c"]), fn.heaviside(0.5, dev["c"]), "heaviside")
-    same(f.heaviside_smooth(ref["a"], 1e-2), fn.heaviside_smooth(dev["a"], 1e-2), "heaviside_smooth")
-    same(f.characteristic_function(1e-10, ref["c"]), fn.characteristic_function(1e-10, dev["c"]), "characteristic")
-    same(f.maximum(ref["a"], ref["b"]), fn.maximum(dev["a"], dev["b"]), "maximum ad/ad")
-    same(f.maximum(ref["a"], cs["b"][0]), fn.maximum(dev["a"], cs["b"][0]), "maximum ad/array")
-    same(f.maximum(cs["b"][0], ref["a"]), fn.maximum(cs["b"][0], dev["a"]), "maximum array/ad")
-    same(f.maximum(ref["a"], 0.1), fn.maximum(dev["a"], 0.1), "maximum ad/scalar")
-    same(f.l2_norm(3, ref["c"]), fn.l2_norm(3, dev["c"]), "l2_norm")
-    same(f.l2_norm(1, ref["a"]), fn.l2_norm(1, dev["a"]), "l2_norm dim 1")
+            d = abs(rj - sps.csr_matrix(gj))
+            assert (d.max() if d.nnz else 0.0) <= 1e-12 * max(abs(rj).max(), 1.0), what
+        checked.add(what)
+    same("exp", fn.exp(dev["a"]))
+    same("log", fn.log(dev["pos"]))
+    same("abs", fn.abs(dev["a"]))
+    same("sin", fn.sin(dev["a"]))
+    same("cos", fn.cos(dev["a"]))
+    same("tanh", fn.tanh(dev["a"]))
+    same("pow", fn.power(dev["pos"], 2.5))
+    same("sqrt", fn.sqrt(dev["pos"]))
+    same("heaviside", fn.heaviside(0.5, dev["c"]))
+    same("heaviside_smooth", fn.heaviside_smooth(dev["a"], 1e-2))
+    same("characteristic", fn.characteristic_function(1e-10, dev["c"]))
+    same("maximum_ad_ad", fn.maximum(dev["a"], dev["b"]))
+    same("maximum_ad_array", fn.maximum(dev["a"], cs["b"][0]))
+    same("maximum_array_ad", fn.maximum(cs["b"][0], dev["a"]))
+    same("maximum_ad_scalar", fn.maximum(dev["a"], 0.1))
+    same("l2_norm", fn.l2_norm(3, dev["c"]))
+    same("l2_norm_dim1", fn.l2_norm(1, dev["a"]))
     # compositions of the kind the friction law uses: b (f_max - ||t||) clipped at zero
-    r = f.maximum(ref["pos"] - f.l2_norm(3, ref["c"]).val.mean(), 0.0) * f.exp(ref["a"])
-    g = fn.maximum(dev["pos"] - float(f.l2_norm(3, ref["c"]).val.mean()), 0.0) * fn.exp(dev["a"])
-    same(r, g, "composition")
+    g = fn.maximum(dev["pos"] - float(ref["l2_norm"][0].mean()), 0.0) * fn.exp(dev["a"])
+    same("composition", g)
+    assert checked == set(ref)
 
 
-@pytest.mark.skipif(not reference_available(), reason="reference tree not present")
 def test_functions_match_the_reference_host_build(monkeypatch):
     import torch
     import emu_sparse
     from porepy_b200 import ad, ad_functions
     emu_sparse.install(monkeypatch)
-    pp = load_porepy()
 
     def make(v, j):
         return ad.DeviceAdArray(torch.as_tensor(v.copy()), emu_sparse.HostCsr(j))
@@ -79,4 +86,4 @@ def test_functions_match_the_reference_host_build(monkeypatch):
         if isinstance(g, ad.DeviceAdArray):
             return g.val.numpy(), g.jac.to_scipy()
         return g.numpy(), None
-    run_checks(make, ad_functions, to_host, pp)
+    run_checks(make, ad_functions, to_host)

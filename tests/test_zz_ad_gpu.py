@@ -1,7 +1,9 @@
 """Device-side forward-mode AD chain (porepy_b200/ad.py, csrc/sparse_ops.cu): SpGEMM / sparse add / diagonal scaling /
-block concatenation against scipy, ``DeviceAdArray`` against the reference's own ``AdArray`` (oracle/_ref when it is on
-the box, else the same formulas on scipy), and a coupled Biot system assembled on the device from the device-resident
-outputs of ``discretize`` against the host assembly (Jacobian entrywise, right-hand side, Newton update)."""
+block concatenation against scipy, ``DeviceAdArray`` against the reference's own ``AdArray`` (stored results), and a
+coupled Biot system assembled on the device from the device-resident outputs of ``discretize`` against the host
+assembly (Jacobian entrywise, right-hand side, Newton update)."""
+import os
+
 import numpy as np
 import pytest
 import scipy.sparse as sps
@@ -57,66 +59,33 @@ def test_sparse_kernels_match_scipy():
     assert _close(D1 @ D2, DeviceCsr(D1).matmul(DeviceCsr(D2)).to_scipy())
 
 
-class _HostAd:
-    """The reference's AdArray formulas on scipy (used when oracle/_ref is not on the box)."""
-
-    def __init__(self, val, jac):
-        self.val, self.jac = np.asarray(val, float), sps.csr_matrix(jac)
-
-    def __add__(self, o):
-        return _HostAd(self.val + o.val, self.jac + o.jac) if isinstance(o, _HostAd) else _HostAd(self.val + o, self.jac)
-
-    def __sub__(self, o):
-        return _HostAd(self.val - o.val, self.jac - o.jac) if isinstance(o, _HostAd) else _HostAd(self.val - o, self.jac)
-
-    def __neg__(self):
-        return _HostAd(-self.val, -self.jac)
-
-    def __mul__(self, o):
-        if isinstance(o, _HostAd):
-            return _HostAd(self.val * o.val, sps.diags(o.val) @ self.jac + sps.diags(self.val) @ o.jac)
-        if np.isscalar(o):
-            return _HostAd(self.val * o, self.jac * o)
-        return _HostAd(self.val * o, sps.diags(o) @ self.jac)
-
-    def __rmatmul__(self, m):
-        return _HostAd(m @ self.val, m @ self.jac)
+GOLDEN_ADARRAY = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ad_adarray.npz")
 
 
-def _reference_adarray():
-    try:
-        from oracle.ref_loader import load_porepy, reference_available
-        if reference_available():
-            return load_porepy().ad.AdArray
-    except Exception:
-        pass
-    return None
-
-
-def test_device_adarray_matches_the_reference_adarray():
+def adarray_case():
+    """Two variables, the operators and the weights of the expression of
+    ``test_device_adarray_matches_the_reference_adarray``."""
     rng = np.random.default_rng(0)
     n1, n2 = 40, 25
     v1, v2 = rng.standard_normal(n1), rng.standard_normal(n2)
     M = _rand(30, n1, 0.2, 11)
     N = _rand(30, n2, 0.3, 12)
     w = rng.standard_normal(30)
+    return v1, v2, M, N, w
+
+
+def test_device_adarray_matches_the_reference_adarray():
+    """The expression evaluated by the reference's own ``AdArray`` is stored in tests/golden/ad_adarray.npz
+    (tools/make_ad_functions_golden.py)."""
+    v1, v2, M, N, w = adarray_case()
     x1, x2 = ad.variables([v1, v2])
     expr = (M @ x1) * (N @ x2) + 3.0 * (M @ x1) - (N @ x2) * w + 2.5
     expr = -expr + (M @ x1) * (M @ x1)
-    Ref = _reference_adarray()
-    J1 = sps.hstack([sps.identity(n1), sps.csr_matrix((n1, n2))]).tocsr()
-    J2 = sps.hstack([sps.csr_matrix((n2, n1)), sps.identity(n2)]).tocsr()
-    if Ref is not None:
-        h1, h2 = Ref(v1, J1), Ref(v2, J2)
-        ref = (M @ h1) * (N @ h2) + 3.0 * (M @ h1) - (N @ h2) * w + 2.5
-        ref = -ref + (M @ h1) * (M @ h1)
-    else:
-        h1, h2 = _HostAd(v1, J1), _HostAd(v2, J2)
-        ref = (M @ h1) * (N @ h2) + (M @ h1) * 3.0 - (N @ h2) * w + 2.5
-        ref = -ref + (M @ h1) * (M @ h1)
+    d = np.load(GOLDEN_ADARRAY)
+    ref_jac = sps.csr_matrix((d["jac__data"], d["jac__indices"], d["jac__indptr"]), shape=tuple(d["jac__shape"]))
     val, jac = expr.host()
-    assert np.allclose(val, ref.val, rtol=1e-13, atol=1e-13)
-    assert _close(ref.jac, jac)
+    assert np.allclose(val, d["val"], rtol=1e-13, atol=1e-13)
+    assert _close(ref_jac, jac)
 
 
 def test_biot_system_assembled_on_the_device():

@@ -98,7 +98,7 @@ def _worker(rank, world, port, q):
     dist.destroy_process_group()
 
 
-@pytest.mark.skipif(_ngpu() < 2, reason="needs two GPUs (gpurun --gpus 2)")
+@pytest.mark.skipif(_ngpu() < 2, reason="needs two GPUs")
 def test_two_gpu_sharded_assembly_halo_exchange_and_fused_solve():
     import torch.multiprocessing as mp
     ctx = mp.get_context("spawn")

@@ -96,11 +96,8 @@ def test_mass_and_energy_balance_on_a_network_gpu(name):
 
 @pytest.mark.gpu
 def test_ad_functions_gpu():
-    """``porepy_b200.ad_functions`` on the device against the reference's ``pp.ad.functions`` (oracle/_ref on the box)."""
+    """``porepy_b200.ad_functions`` on the device against the reference's ``pp.ad.functions`` (tests/golden/ad_functions.npz)."""
     import torch
-    from oracle.ref_loader import load_porepy, reference_available
-    if not reference_available():
-        pytest.skip("the reference is not on this box")
     from porepy_b200 import ad, ad_functions
     from porepy_b200.sparse import DeviceCsr
     from test_ad_functions import run_checks
@@ -112,7 +109,7 @@ def test_ad_functions_gpu():
         if isinstance(g, ad.DeviceAdArray):
             return g.val.cpu().numpy(), g.jac.to_scipy()
         return g.cpu().numpy(), None
-    run_checks(make, ad_functions, to_host, load_porepy())
+    run_checks(make, ad_functions, to_host)
 
 
 @pytest.mark.gpu

@@ -3,4 +3,4 @@ import os
 import sys
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-from oracle.ref_loader import REF_SRC, load_porepy, reference_available  # noqa: E402,F401
+from oracle.ref_loader import REF_SRC, REF_TESTS, load_porepy, reference_available  # noqa: E402,F401

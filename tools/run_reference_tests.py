@@ -1,7 +1,7 @@
 """Run the REFERENCE's own finite-volume unit tests (tests/numerics/fv/test_{mpfa,mpsa,biot}.py of the
 read-only tree) with pp.Mpfa / pp.Mpsa / pp.Biot rebound to the porepy_b200 plugin classes.
 
-    python tools/run_reference_tests.py            # build container or any box with /root/reference
+    python tools/run_reference_tests.py            # wherever the reference (or its copy under oracle/_ref) is
     python tools/run_reference_tests.py functional/test_terzaghi.py [--stock] [pytest options]
 
 With a GPU the plugin runs the CUDA path; without one the device plan is replaced by the host build of the
@@ -17,7 +17,6 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 for p in (ROOT, os.path.join(ROOT, "tools"), os.path.join(ROOT, "tests")):
     if p not in sys.path:
         sys.path.insert(0, p)
-REF_TESTS = "/root/reference/tests/numerics/fv"
 COUNTS = collections.Counter()
 
 
@@ -67,15 +66,16 @@ class Rebind:
 
 if __name__ == "__main__":
     import pytest
-    if not os.path.isdir(REF_TESTS):
-        sys.exit("reference tree not present")
-    # extra arguments: reference test files (relative to /root/reference/tests) and pytest options
+    from ref_loader import REF_TESTS
+    if REF_TESTS is None:
+        sys.exit("reference tests not present (run oracle/make_ref.sh)")
+    # extra arguments: reference test files (relative to the reference's tests/) and pytest options
     extra = [a for a in sys.argv[1:] if a.endswith(".py") or "::" in a]
     opts = [a for a in sys.argv[1:] if a not in extra and a != "--stock"]
     if extra:
-        files = [os.path.join("/root/reference/tests", a) for a in extra]
+        files = [os.path.join(REF_TESTS, a) for a in extra]
     else:
-        files = [os.path.join(REF_TESTS, f) for f in ("test_mpfa.py", "test_mpsa.py", "test_biot.py")]
+        files = [os.path.join(REF_TESTS, "numerics", "fv", f) for f in ("test_mpfa.py", "test_mpsa.py", "test_biot.py")]
     os.chdir("/tmp")
     sys.exit(pytest.main(files + ["-p", "no:cacheprovider", "-o", "addopts=", "-q", "--rootdir", "/tmp", *opts],
                          plugins=[Rebind()]))
