@@ -344,6 +344,37 @@ int pb_csr_block_diag_inv_dev(const pb_csr *a, int bs, int64_t nblocks, double *
 int pb_kry_xr(int64_t n, double *x, const double *ph, const double *sh, const double *s, const double *t, double *r,
               const double *rhat, double *scal, int cur, int carry /* 1 on exactly one rank */, uint64_t stream);
 
+/* ---- local-block inverse preconditioner (csrc/local_blocks.cu).  A layout partitions rows and columns of a square
+ * matrix into nblocks blocks: block b pairs rows[blk_ptr[b] .. blk_ptr[b+1]) with cols[same range], s_b <= 32.
+ * inv_ptr: prefix sums of s_b^2 (nblocks + 1); order: the block ids grouped by team size (s_b <= 4, 8, 16, 32), with the
+ * HOST array class_ptr[5] delimiting the four groups.  All other pointers are DEVICE pointers.
+ * Factorisation: inv[inv_ptr[b] ..] = A[rows_b, cols_b]^-1, row-major, by Gauss-Jordan with partial pivoting (FP64).
+ * A non-finite entry, a pivot that is not finite or <= 1e-14 max|B_b|, or a non-finite inverse returns PB_ESINGULAR
+ * naming the first failing block (err_dev: one device word of scratch; the call synchronises the stream once to read it).
+ * Application: z[cols_b] = B_b^-1 r[rows_b] for every block, one launch per team size; skip: NULL or a device double,
+ * when it is non-zero the call does nothing (the sticky DONE flag of the GMRES loop). */
+int pb_csr_local_block_inv_dev(const pb_csr *a, int64_t nblocks, const int64_t *blk_ptr, const int32_t *rows,
+                               const int32_t *cols, const int64_t *inv_ptr, const int32_t *order,
+                               const int64_t *class_ptr, double *inv, uint64_t *err_dev, uint64_t stream);
+int pb_local_block_apply_dev(int64_t nblocks, const int64_t *blk_ptr, const int32_t *rows, const int32_t *cols,
+                             const int64_t *inv_ptr, const int32_t *order, const int64_t *class_ptr, const double *inv,
+                             const double *r, double *z, const double *skip, uint64_t stream);
+
+/* ---- vector kernels of the restarted right-preconditioned GMRES(m) with CGS2 (csrc/gmres.cu).  V: n x (m+1) basis,
+ * column-major; H: (m+1) x m Hessenberg matrix, column-major; hb: 2 (m+1) + 2 doubles (two Gram-Schmidt passes and
+ * their ||w||^2); scal: the 8-double scalar buffer described in gmres.cu.  All pointers are DEVICE pointers. */
+int pb_gm_dots(int64_t n, const double *V, int ncols, const double *w, double *h, const double *scal, uint64_t stream);
+int pb_gm_orth(int64_t n, const double *V, int ncols, const double *h, double *w, double *ww, const double *scal,
+               uint64_t stream);
+int pb_gm_givens(int j, int m, double *H, double *hb, double *cs, double *sn, double *g, double *scal, uint64_t stream);
+int pb_gm_scale(int64_t n, double *v, const double *scal, uint64_t stream);
+int pb_gm_residual(int64_t n, const double *b, double *r, double *scal, int with_bb, uint64_t stream);
+int pb_gm_start(int m, double tol, double *hb, double *g, double *scal, uint64_t stream);
+int pb_gm_ysolve(int m, const double *H, const double *g, double *y, const double *scal, uint64_t stream);
+int pb_gm_combine(int64_t n, const double *V, int m, const double *y, double *t, const double *scal, int accumulate,
+                  uint64_t stream);
+int pb_gm_axpy(int64_t n, const double *z, double *x, uint64_t stream);
+
 /* time `reps` device SpMVs with CUDA events on the launching stream; returns mean ms */
 int pb_csr_spmv_bench(pb_csr *a, int reps, float *mean_ms);
 

@@ -99,6 +99,18 @@ _SIGNATURES = {
     "pb_csr_block_diag_inv_dev": (C.c_int, [C.c_void_p, C.c_int, C.c_int64, C.c_void_p, C.c_uint64]),
     "pb_kry_xr": (C.c_int, [C.c_int64] + [C.c_void_p] * 8 + [C.c_int, C.c_int, C.c_uint64]),
     "pb_csr_spmv_bench": (C.c_int, [C.c_void_p, C.c_int, _f32p]),
+    "pb_csr_local_block_inv_dev": (C.c_int, [C.c_void_p, C.c_int64] + [C.c_void_p] * 5 + [_i64p, C.c_void_p, C.c_void_p,
+                                                                                         C.c_uint64]),
+    "pb_local_block_apply_dev": (C.c_int, [C.c_int64] + [C.c_void_p] * 5 + [_i64p] + [C.c_void_p] * 4 + [C.c_uint64]),
+    "pb_gm_dots": (C.c_int, [C.c_int64, C.c_void_p, C.c_int] + [C.c_void_p] * 3 + [C.c_uint64]),
+    "pb_gm_orth": (C.c_int, [C.c_int64, C.c_void_p, C.c_int] + [C.c_void_p] * 4 + [C.c_uint64]),
+    "pb_gm_givens": (C.c_int, [C.c_int, C.c_int] + [C.c_void_p] * 6 + [C.c_uint64]),
+    "pb_gm_scale": (C.c_int, [C.c_int64, C.c_void_p, C.c_void_p, C.c_uint64]),
+    "pb_gm_residual": (C.c_int, [C.c_int64] + [C.c_void_p] * 3 + [C.c_int, C.c_uint64]),
+    "pb_gm_start": (C.c_int, [C.c_int, C.c_double] + [C.c_void_p] * 3 + [C.c_uint64]),
+    "pb_gm_ysolve": (C.c_int, [C.c_int] + [C.c_void_p] * 4 + [C.c_uint64]),
+    "pb_gm_combine": (C.c_int, [C.c_int64, C.c_void_p, C.c_int] + [C.c_void_p] * 3 + [C.c_int, C.c_uint64]),
+    "pb_gm_axpy": (C.c_int, [C.c_int64, C.c_void_p, C.c_void_p, C.c_uint64]),
 }
 
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)

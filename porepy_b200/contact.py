@@ -20,8 +20,10 @@ with the displacement jump ``[u] = R Pi^avg_{mortar -> fracture} S u_j`` (``S``:
 coordinates; constitutive_laws.py ``displacement_jump``).  ``maximum`` / ``l2_norm`` / ``characteristic_function`` are those of
 ``porepy_b200.ad_functions`` with the reference's tie rules, so the Jacobian of the semismooth laws is the reference's.  The
 elastic fracture-deformation laws (Barton-Bandis closure, tangential stiffness) are off in the reference's defaults and not
-stated here.  The Jacobian has zeros on the diagonal of the complementarity rows: ``time_step`` takes the linear solver from
-the caller (the tests use a direct solve); a device Krylov method for this saddle-point system is future work.
+stated here.  The Jacobian has zeros on the diagonal of the complementarity rows, so point and 3 x 3 Jacobi are undefined:
+``device_linear_solver`` solves the Newton steps on the device with restarted GMRES preconditioned by the inverses of the
+local blocks of ``block_layout`` (one per matrix cell, one per fracture cell with its two mortar cells); ``time_step``
+takes any ``linear_solver(J, rhs) -> dx``.
 ``tests/golden/contact_model.npz`` pins Jacobian, residual, residual history and the converged sliding state.
 """
 from __future__ import annotations
@@ -54,6 +56,83 @@ class FractureContact:
         self.rotation = sps.csr_matrix(local_coordinates)
         self.num_mortar = int(np.asarray(mortar_sign).size)
         self.num_cells = int(self.rotation.shape[0] // 3)
+        self.mortar_to_secondary = sps.csr_matrix(mortar_to_secondary_avg)
+
+
+def mortar_pairs(mortar_to_secondary) -> np.ndarray:
+    """(num fracture cells, 2): the two mortar cells of every fracture cell, from the scalar mortar -> fracture
+    projection.  A fracture cell without exactly two mortar cells (an intersection, a one-sided interface) has no
+    local block of the kind ``local_block_layout`` builds."""
+    m2s = sps.csr_matrix(mortar_to_secondary, copy=True)
+    m2s.eliminate_zeros()
+    m2s.sort_indices()
+    if np.any(np.diff(m2s.indptr) != 2):
+        raise NotImplementedError("local blocks need exactly two mortar cells per fracture cell")
+    return m2s.indices.reshape(-1, 2).astype(np.int64)
+
+
+def local_block_layout(num_cells: int, pairs, cell_unknowns, cell_equations, fracture_unknowns, fracture_equations):
+    """The local blocks of a contact model's Jacobian, from the model's own offsets: one block per matrix cell (its
+    ``cell_unknowns`` / ``cell_equations``: lists of (offset, width): entries offset + width * cell + 0..width-1) and one
+    per fracture cell (``fracture_unknowns[j]`` / ``fracture_equations[j]`` of fracture j: lists of (offset, width, on),
+    ``on`` = "fracture" for a field per fracture cell, "mortar" for a field per mortar cell: both mortar cells of the
+    fracture cell, ``pairs[j]``, go into its block).  Returns ``SimpleNamespace(ptr, rows, cols)``: every row and every
+    column of the Jacobian belongs to exactly one block (asserted)."""
+    def take(fields, ids_of):
+        return np.hstack([(off + ids_of[on][:, :, None] * w + np.arange(w)).reshape(ids_of[on].shape[0], -1)
+                          for off, w, on in fields])
+    cells = {"cell": np.arange(num_cells, dtype=np.int64)[:, None]}
+    rows = [take([(o, w, "cell") for o, w in cell_equations], cells)]
+    cols = [take([(o, w, "cell") for o, w in cell_unknowns], cells)]
+    for pr, fu, fe in zip(pairs, fracture_unknowns, fracture_equations):
+        pr = np.asarray(pr, np.int64)
+        ids = {"fracture": np.arange(pr.shape[0], dtype=np.int64)[:, None], "mortar": pr}
+        rows.append(take(fe, ids))
+        cols.append(take(fu, ids))
+    for r, c in zip(rows, cols):
+        assert r.shape == c.shape, "a block needs as many equations as unknowns"
+    sizes = np.concatenate([np.full(r.shape[0], r.shape[1], np.int64) for r in rows])
+    layout = SimpleNamespace(ptr=np.concatenate(([0], np.cumsum(sizes))).astype(np.int64),
+                             rows=np.concatenate([r.ravel() for r in rows]), cols=np.concatenate([c.ravel() for c in cols]))
+    n = layout.rows.size
+    assert np.array_equal(np.bincount(layout.rows, minlength=n), np.ones(n, np.int64)), "rows: not a bijection"
+    assert np.array_equal(np.bincount(layout.cols, minlength=n), np.ones(n, np.int64)), "columns: not a bijection"
+    return layout
+
+
+def offsets_of(sizes) -> np.ndarray:
+    return np.concatenate(([0], np.cumsum(sizes))).astype(np.int64)
+
+
+class DeviceLinearSolver:
+    """``linear_solver(J, rhs) -> dx`` of the models' ``time_step`` on the device: the local blocks of ``J``
+    (``problem.block_layout()``, uploaded on the first call) are inverted at every call and GMRES
+    (``krylov.gmres``) runs with them as right preconditioner; its info goes to ``history``.  Raises ``RuntimeError``
+    when GMRES does not reach ``tol``."""
+
+    def __init__(self, problem, tol: float = 1e-12, restart: int = 100, maxiter: int = 2000):
+        self.layout = problem.block_layout()
+        self.tol, self.restart, self.maxiter = float(tol), int(restart), int(maxiter)
+        self.blocks = None
+        self.history = []
+
+    def __call__(self, J, rhs):
+        from . import krylov
+        if self.blocks is None:
+            self.blocks = krylov.LocalBlocks(self.layout)
+        self.blocks.factor(J)
+        dx, info = krylov.gmres(J, rhs, precond=self.blocks, tol=self.tol, restart=self.restart, maxiter=self.maxiter)
+        self.history.append(info)
+        if not info["converged"]:
+            raise RuntimeError(f"GMRES did not converge: {info['iterations']} iterations, relative residual "
+                               f"{info['relres']:.3e} (tol {self.tol:.1e})")
+        return dx
+
+
+def device_linear_solver(problem, tol: float = 1e-12, restart: int = 100, maxiter: int = 2000) -> DeviceLinearSolver:
+    """The device solve of the Newton steps of ``problem`` (a contact model with ``block_layout()``), for its
+    ``time_step(..., linear_solver=...)``."""
+    return DeviceLinearSolver(problem, tol, restart, maxiter)
 
 
 class FracturedMomentumBalance:
@@ -85,6 +164,20 @@ class FracturedMomentumBalance:
     def discretize(self) -> None:
         Mpsa(self.kw).discretize(self.sd, self.data)
         self._const = None
+
+    def block_layout(self):
+        """Local blocks of the Jacobian: u of every matrix cell (3), and per fracture cell its traction with the u_j of
+        its two mortar cells (9), paired with the momentum balance, resp. the normal and tangential laws and the two
+        force balances."""
+        nfr = len(self.fractures)
+        o = self.offsets
+        e = offsets_of([3 * self.nc] + [3 * f.num_mortar for f in self.fractures] + [f.num_cells for f in self.fractures]
+                       + [2 * f.num_cells for f in self.fractures])
+        return local_block_layout(
+            self.nc, [mortar_pairs(f.mortar_to_secondary) for f in self.fractures], [(o[0], 3)], [(e[0], 3)],
+            [[(o[1 + j], 3, "fracture"), (o[1 + nfr + j], 3, "mortar")] for j in range(nfr)],
+            [[(e[1 + nfr + j], 1, "fracture"), (e[1 + 2 * nfr + j], 2, "fracture"), (e[1 + j], 3, "mortar")]
+             for j in range(nfr)])
 
     def _operands(self):
         if self._const is None:
@@ -147,7 +240,8 @@ class FracturedMomentumBalance:
         return ad.assemble(self.equations(x, x_prev))
 
     def time_step(self, x_prev, linear_solver, x0=None, tol: float = 1e-10, max_iterations: int = 30, verbose: bool = False):
-        """Semismooth Newton from ``x0`` (default: the previous state); ``linear_solver(J, rhs) -> dx``."""
+        """Semismooth Newton from ``x0`` (default: the previous state); ``linear_solver(J, rhs) -> dx``, e.g.
+        ``device_linear_solver(self)``."""
         import torch
         x_prev = ad.device_vector(x_prev)
         x = x_prev.clone() if x0 is None else ad.device_vector(x0).clone()

@@ -19,8 +19,9 @@ fracture flux is RE-DISCRETIZED in front of every linearization with the tangent
 aperture (``operator_to_SecondOrderTensor``: the specific volume of the iterate; not differentiated), next to the
 upwinding.  Unknowns: [p matrix | p fractures | u | contact tractions | lambda | u_j]; equations:
 [mass matrix | mass fractures | momentum | Darcy laws | force balances | normal laws | tangential laws] (the fixtures carry
-the maps to the reference's numbering).  One matrix subdomain, fractures without intersections; saddle-point Jacobian: the
-linear solver of ``time_step`` is the caller's.  ``tests/golden/contact_poromech*.npz`` pin Jacobian, residual, the residual
+the maps to the reference's numbering).  One matrix subdomain, fractures without intersections; saddle-point Jacobian:
+``contact.device_linear_solver`` solves the Newton steps on the device (GMRES with the local blocks of ``block_layout``),
+and ``time_step`` takes any ``linear_solver(J, rhs) -> dx``.  ``tests/golden/contact_poromech*.npz`` pin Jacobian, residual, the residual
 history of the semismooth Newton loop and the converged state.
 """
 from __future__ import annotations
@@ -31,6 +32,7 @@ import numpy as np
 import scipy.sparse as sps
 
 from . import ad, ad_functions as fn
+from .contact import local_block_layout, mortar_pairs, offsets_of
 from .fv import Biot, Mpfa, Upwind, UpwindCoupling
 from .params import DISCRETIZATION_MATRICES, PARAMETERS
 
@@ -88,6 +90,22 @@ class FracturedPoromechanics:
     @property
     def num_dofs(self) -> int:
         return int(self.offsets[-1])
+
+    def block_layout(self):
+        """Local blocks of the Jacobian: p and u of every matrix cell (4, with the mass and momentum balances), and per
+        fracture cell its traction and pressure with lambda and u_j of its two mortar cells (12, with the fracture mass
+        balance, the contact laws and the Darcy laws and force balances of the two mortar cells)."""
+        nfr, o = len(self.fractures), self.offsets
+        nfc = [f.num_cells for f in self.fractures]
+        nm = [f.num_mortar for f in self.fractures]
+        e = offsets_of([self.nc] + nfc + [3 * self.nc] + nm + [3 * n for n in nm] + nfc + [2 * n for n in nfc])
+        return local_block_layout(
+            self.nc, [mortar_pairs(f.p["mortar_to_secondary_avg"]) for f in self.fractures],
+            [(o[0], 1), (o[1 + nfr], 3)], [(e[0], 1), (e[1 + nfr], 3)],
+            [[(o[2 + nfr + j], 3, "fracture"), (o[1 + j], 1, "fracture"), (o[2 + 2 * nfr + j], 1, "mortar"),
+              (o[2 + 3 * nfr + j], 3, "mortar")] for j in range(nfr)],
+            [[(e[2 + 3 * nfr + j], 1, "fracture"), (e[2 + 4 * nfr + j], 2, "fracture"), (e[1 + j], 1, "fracture"),
+              (e[2 + nfr + j], 1, "mortar"), (e[2 + 2 * nfr + j], 3, "mortar")] for j in range(nfr)])
 
     def _discretize_fracture(self, fc, aperture) -> None:
         from .params import SecondOrderTensor
@@ -272,7 +290,8 @@ class FracturedPoromechanics:
         return ad.assemble(self.equations(x, x_prev, dt))
 
     def time_step(self, x_prev, dt: float, linear_solver, tol: float = 1e-10, max_iterations: int = 30, verbose: bool = False):
-        """Semismooth Newton; ``linear_solver(J, rhs) -> dx``.  Returns (x, history)."""
+        """Semismooth Newton; ``linear_solver(J, rhs) -> dx`` (e.g. ``contact.device_linear_solver(self)``).  Returns
+        (x, history)."""
         import torch
         x_prev = ad.device_vector(x_prev)
         x = x_prev.clone()

@@ -15,7 +15,8 @@ fracture's internal energy and in the interface Fourier law:
 
 Unknowns: [p matrix | p fractures | T matrix | T fractures | u | contact tractions | lambda | eta | eps | u_j]; equations:
 [mass matrix | mass fractures | energy matrix | energy fractures | momentum | Darcy laws | Fourier laws | enthalpy laws |
-force balances | normal laws | tangential laws].  ``tests/golden/contact_thm*.npz`` pin the Jacobian at the zero state and at
+force balances | normal laws | tangential laws].  ``contact.device_linear_solver`` solves the Newton steps on the device
+(GMRES with the local blocks of ``block_layout``).  ``tests/golden/contact_thm*.npz`` pin the Jacobian at the zero state and at
 the fourth Newton iterate, the residual history of the semismooth Newton loop and the converged state.
 """
 from __future__ import annotations
@@ -25,6 +26,7 @@ from types import SimpleNamespace
 import numpy as np
 
 from . import ad, ad_functions as fn
+from .contact import local_block_layout, mortar_pairs, offsets_of
 from .fractured_poromech import FracturedPoromechanics
 from .fv import Mpfa, Upwind, UpwindCoupling
 from .params import DISCRETIZATION_MATRICES, PARAMETERS, SecondOrderTensor
@@ -50,6 +52,26 @@ class FracturedThermoporomechanics(FracturedPoromechanics):
         nm = [f.num_mortar for f in self.fractures]
         self.sizes = [self.nc] + nfc + [self.nc] + nfc + [3 * self.nc] + [3 * n for n in nfc] + nm + nm + nm + [3 * n for n in nm]
         self.offsets = np.concatenate(([0], np.cumsum(self.sizes))).astype(np.int64)
+
+    def block_layout(self):
+        """Local blocks of the Jacobian: p, T and u of every matrix cell (5, with the mass, energy and momentum
+        balances), and per fracture cell its traction, pressure and temperature with lambda, eta, eps and u_j of its two
+        mortar cells (17, with the fracture mass and energy balances, the contact laws and the Darcy, Fourier and
+        enthalpy laws and force balances of the two mortar cells)."""
+        nfr, o = len(self.fractures), self.offsets
+        nfc = [f.num_cells for f in self.fractures]
+        nm = [f.num_mortar for f in self.fractures]
+        e = offsets_of([self.nc] + nfc + [self.nc] + nfc + [3 * self.nc] + nm + nm + nm + [3 * n for n in nm] + nfc
+                       + [2 * n for n in nfc])
+        return local_block_layout(
+            self.nc, [mortar_pairs(f.p["mortar_to_secondary_avg"]) for f in self.fractures],
+            [(o[0], 1), (o[1 + nfr], 1), (o[2 + 2 * nfr], 3)], [(e[0], 1), (e[1 + nfr], 1), (e[2 + 2 * nfr], 3)],
+            [[(o[3 + 2 * nfr + j], 3, "fracture"), (o[1 + j], 1, "fracture"), (o[2 + nfr + j], 1, "fracture")]
+             + [(o[3 + q * nfr + j], 1, "mortar") for q in (3, 4, 5)] + [(o[3 + 6 * nfr + j], 3, "mortar")]
+             for j in range(nfr)],
+            [[(e[3 + 6 * nfr + j], 1, "fracture"), (e[3 + 7 * nfr + j], 2, "fracture"), (e[1 + j], 1, "fracture"),
+              (e[2 + nfr + j], 1, "fracture")] + [(e[3 + q * nfr + j], 1, "mortar") for q in (2, 3, 4)]
+             + [(e[3 + 5 * nfr + j], 3, "mortar")] for j in range(nfr)])
 
     # ---- discretizations
     def _matrix_conductivity(self):

@@ -480,3 +480,261 @@ def solve_local(loc: LocalSystem, b_own, diag_own=None, tol: float = 1e-10, maxi
     x, info = bicgstab(op, b, tol=tol, maxiter=maxiter, diag_own=dg, block_inv=block_inv)
     info["halo_bytes_per_spmv"] = op.halo_bytes
     return x, info
+
+
+# ------------------------------------------------------------------------------------------
+# restarted GMRES with a local-block preconditioner: the Newton steps of the contact models
+# ------------------------------------------------------------------------------------------
+
+
+def _size_classes(sizes: np.ndarray):
+    """Block ids grouped by team size (s <= 4, 8, 16, 32) and the five group boundaries."""
+    cls = np.searchsorted(np.array([4, 8, 16, 32]), sizes)           # 0..3 (sizes <= 32 checked by the caller)
+    order = np.argsort(cls, kind="stable").astype(np.int32)
+    ptr = np.concatenate(([0], np.cumsum(np.bincount(cls, minlength=4)))).astype(np.int64)
+    return order, ptr
+
+
+def check_block_layout(layout, n: int | None = None) -> None:
+    """A layout (``ptr``, ``rows``, ``cols``) must pair every row and every column of an n x n matrix with exactly one
+    block, and no block may be wider than 32."""
+    ptr, rows, cols = np.asarray(layout.ptr), np.asarray(layout.rows), np.asarray(layout.cols)
+    n = int(rows.size) if n is None else int(n)
+    sizes = np.diff(ptr)
+    if ptr[0] != 0 or ptr[-1] != rows.size or rows.size != cols.size or np.any(sizes < 1) or np.any(sizes > 32):
+        raise ValueError("block layout: blocks of 1..32 rows and as many columns are expected")
+    for name, ix in (("rows", rows), ("cols", cols)):
+        if ix.size != n or not np.array_equal(np.bincount(ix, minlength=n), np.ones(n, np.int64)):
+            raise ValueError(f"block layout: the {name} are not a bijection onto 0..{n - 1}")
+
+
+class LocalBlocks:
+    """Local-block inverse preconditioner (csrc/local_blocks.cu) on a fixed layout: ``layout.ptr`` (block pointers),
+    ``layout.rows`` / ``layout.cols`` (row and column of every block entry; each a bijection).  The layout is uploaded
+    once; ``factor(J)`` inverts the blocks ``J[rows_b, cols_b]`` of a device matrix (every Newton step), ``apply(r, out)``
+    writes ``out[cols_b] = B_b^-1 r[rows_b]``.  A singular block raises ``ValueError`` naming it; there is no fallback."""
+
+    def __init__(self, layout, device=None):
+        import torch
+        self.torch = torch
+        check_block_layout(layout)
+        ptr = np.asarray(layout.ptr, np.int64)
+        sizes = np.diff(ptr)
+        self.n, self.num_blocks = int(ptr[-1]), int(sizes.size)
+        self.sizes = sizes
+        order, self.class_ptr = _size_classes(sizes)
+        inv_ptr = np.concatenate(([0], np.cumsum(sizes * sizes))).astype(np.int64)
+        dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+        if dev.type != "cuda":
+            raise RuntimeError("porepy_b200.krylov.LocalBlocks: the block kernels need a CUDA device (no CPU path)")
+        up = lambda a, dt: torch.as_tensor(np.ascontiguousarray(a), dtype=dt, device=dev)  # noqa: E731
+        self.ptr, self.inv_ptr = up(ptr, torch.int64), up(inv_ptr, torch.int64)
+        self.rows, self.cols = up(layout.rows, torch.int32), up(layout.cols, torch.int32)
+        self.order = up(order, torch.int32)
+        self.inv = torch.empty(int(inv_ptr[-1]), dtype=torch.float64, device=dev)
+        self.err = torch.zeros(1, dtype=torch.int64, device=dev)
+        self.device = dev
+
+    def _args(self):
+        import ctypes as C
+        P = lambda a: C.c_void_p(a.data_ptr())  # noqa: E731
+        return (self.num_blocks, P(self.ptr), P(self.rows), P(self.cols), P(self.inv_ptr), P(self.order),
+                self.class_ptr.ctypes.data_as(C.POINTER(C.c_int64)))
+
+    def factor(self, J, stream: int = 0) -> "LocalBlocks":
+        import ctypes as C
+        from . import _lib
+        if tuple(J.shape) != (self.n, self.n):
+            raise ValueError(f"LocalBlocks.factor: a {self.n} x {self.n} matrix is expected, got {J.shape}")
+        st = stream or self.torch.cuda.current_stream().cuda_stream
+        _lib.check(_lib.load().pb_csr_local_block_inv_dev(J.h, *self._args(), C.c_void_p(self.inv.data_ptr()),
+                                                          C.c_void_p(self.err.data_ptr()), st))
+        return self
+
+    def apply(self, r, out=None, stream: int = 0, skip=None):
+        """``skip``: a device address (int) of a double; when it holds a non-zero value the call does nothing (the
+        GMRES loop passes its sticky DONE flag)."""
+        import ctypes as C
+        from . import _lib
+        if out is None:
+            out = self.torch.empty(self.n, dtype=self.torch.float64, device=self.device)
+        st = stream or self.torch.cuda.current_stream().cuda_stream
+        _lib.check(_lib.load().pb_local_block_apply_dev(*self._args(), C.c_void_p(self.inv.data_ptr()),
+                                                        C.c_void_p(r.data_ptr()), C.c_void_p(out.data_ptr()),
+                                                        None if skip is None else C.c_void_p(skip), st))
+        return out
+
+
+def _matvec_of(a):
+    if hasattr(a, "matvec"):
+        return a.matvec
+    return lambda v: a @ v
+
+
+def gmres(a, b, precond=None, x0=None, tol: float = 1e-12, restart: int = 100, maxiter: int = 2000,
+          check_every: int = 8):
+    """Restarted right-preconditioned GMRES(m) with classical Gram-Schmidt and one reorthogonalisation pass (CGS2).
+    ``a``: ``DeviceCsr`` or an operator with ``matvec``; ``b``: a tensor; ``precond``: an object with
+    ``apply(r, out)`` (``LocalBlocks``) or None.  Single process.  Returns (x, info), info = {"iterations" (Arnoldi
+    steps), "restarts", "relres" (the TRUE residual ||b - A x|| / ||b||, recomputed at every restart and before
+    convergence is reported), "converged" (relres <= tol), "host_syncs"}.
+    With a ``DeviceCsr`` the device loop runs (``_gmres_fused``: all scalars on the device, one host read per
+    ``check_every`` steps and one per restart); it takes a ``LocalBlocks`` preconditioner or none, any other raises
+    ``TypeError``.  Otherwise the eager torch recurrence below runs, the same algorithm, which the CPU tests run on a
+    matvec stand-in; it reads the Hessenberg column once per step, so its ``host_syncs`` is one per step plus one per
+    restart (and one for ||b||)."""
+    from .sparse import DeviceCsr
+    if isinstance(a, DeviceCsr):
+        if precond is not None and not isinstance(precond, LocalBlocks):
+            raise TypeError("gmres: the device loop takes a krylov.LocalBlocks preconditioner or none, "
+                            f"not {type(precond).__name__}")
+        return _gmres_fused(a, b, precond, x0, tol, restart, maxiter, check_every)
+    import torch
+    mv = _matvec_of(a)
+    n = b.numel()
+    m = max(1, min(int(restart), n))
+    x = torch.zeros_like(b) if x0 is None else x0.clone()
+    bnorm = float(torch.linalg.vector_norm(b))
+    syncs = 1
+    if bnorm == 0.0:
+        return torch.zeros_like(b), {"iterations": 0, "restarts": 0, "relres": 0.0, "converged": True, "host_syncs": syncs}
+    prec = (lambda v: v) if precond is None else (lambda v: precond.apply(v, torch.empty_like(v)))  # noqa: E731
+    V = torch.zeros(m + 1, n, dtype=b.dtype, device=b.device)
+    H = np.zeros((m + 1, m))
+    it, cycles, relres = 0, 0, 1.0
+    while True:
+        r = b - mv(x)
+        beta = float(torch.linalg.vector_norm(r))
+        syncs += 1
+        relres = beta / bnorm
+        if not np.isfinite(relres) or relres <= tol or it >= maxiter:
+            break
+        V[0] = r / beta
+        g = np.zeros(m + 1)
+        g[0] = beta
+        cs, sn = np.zeros(m), np.zeros(m)
+        k = 0
+        for j in range(min(m, maxiter - it)):
+            w = mv(prec(V[j]))
+            h = torch.zeros(j + 1, dtype=b.dtype, device=b.device)
+            for _ in range(2):                                     # CGS2
+                hp = V[:j + 1] @ w
+                w = w - V[:j + 1].T @ hp
+                h = h + hp
+            hv = torch.cat((h, torch.linalg.vector_norm(w).reshape(1))).cpu().numpy()     # one host read per step
+            syncs += 1
+            hn = float(hv[-1])
+            col = np.zeros(m + 1)
+            col[:j + 1] = hv[:-1]
+            for i in range(j):
+                col[i], col[i + 1] = cs[i] * col[i] + sn[i] * col[i + 1], -sn[i] * col[i] + cs[i] * col[i + 1]
+            rr = float(np.hypot(col[j], hn))
+            cs[j], sn[j] = (col[j] / rr, hn / rr) if rr > 0 else (1.0, 0.0)
+            col[j], col[j + 1] = rr, 0.0
+            g[j + 1], g[j] = -sn[j] * g[j], cs[j] * g[j]
+            H[:, j] = col
+            k = j + 1
+            if not abs(g[j + 1]) > tol * bnorm or not hn > 1e-15 * rr:
+                break
+            V[j + 1] = w / hn
+        it += k
+        cycles += 1
+        y = np.zeros(k)
+        for i in range(k - 1, -1, -1):
+            y[i] = (g[i] - H[i, i + 1:k] @ y[i + 1:k]) / H[i, i]
+        x = x + prec(V[:k].T @ torch.as_tensor(y, dtype=b.dtype, device=b.device))
+        if k == 0:
+            break
+    return x, {"iterations": it, "restarts": max(cycles - 1, 0), "relres": relres, "converged": bool(relres <= tol),
+               "host_syncs": syncs}
+
+
+def _gmres_fused(a, b, precond, x0, tol, restart, maxiter, check_every):
+    """The GMRES loop on the device (csrc/gmres.cu): plain launches, no CUDA graph (the multi-column kernels change
+    their width every step).  The host reads the scalar buffer once per ``check_every`` Arnoldi steps and once per
+    restart (the true residual).  Once the DONE flag is set inside a block of steps, every GMRES kernel and the block
+    apply of the remaining steps return at once; the SpMV (the shared ``pb_csr_spmv_dev``) does not read the flag, so
+    up to ``check_every - 1`` SpMVs per solve run for nothing -- at most 7 against the 450-1800 steps of the measured
+    contact problems."""
+    import ctypes as C
+    import torch
+    from . import _lib
+    lib = _lib.load()
+    n = int(a.shape[0])
+    if tuple(a.shape) != (n, n) or b.numel() != n:
+        raise ValueError("gmres: a square matrix and a right-hand side of matching size are expected")
+    if not b.is_cuda:
+        raise RuntimeError("gmres: the device loop needs a CUDA right-hand side (no CPU path)")
+    if precond is not None and precond.n != n:
+        raise ValueError("gmres: the preconditioner's layout does not match the matrix")
+    dev = b.device
+    m = max(1, min(int(restart), n, 4096))
+    check_every = max(1, int(check_every))
+    b = b.contiguous().to(torch.float64)
+    f64 = lambda k: torch.zeros(k, dtype=torch.float64, device=dev)  # noqa: E731
+    x = f64(n) if x0 is None else x0.to(torch.float64).clone().contiguous()
+    V = torch.zeros((m + 1) * n, dtype=torch.float64, device=dev)
+    z, t = f64(n), f64(n)
+    H, hb, cs, sn, g, y = f64((m + 1) * m), f64(2 * (m + 1) + 2), f64(m), f64(m), f64(m + 1), f64(m)
+    scal = f64(8)
+    done = C.c_void_p(scal.data_ptr() + 8 * 5)                     # the sticky DONE flag (GS_DONE in gmres.cu)
+    P = lambda q: C.c_void_p(q.data_ptr())  # noqa: E731
+    A = lambda off: C.c_void_p(V.data_ptr() + 8 * off)  # noqa: E731
+    col = lambda j: A(j * n)  # noqa: E731
+    st = torch.cuda.current_stream().cuda_stream
+    ck = _lib.check
+    syncs, it, cycles, relres, bnorm = 0, 0, 0, 1.0, None
+    v0 = V[:n]
+    while True:
+        # true residual r = b - A x into V[:, 0]
+        scal[1].zero_()
+        a.spmv_device(x.data_ptr(), V.data_ptr(), st)
+        ck(lib.pb_gm_residual(n, P(b), P(V), P(scal), int(bnorm is None), st))
+        ck(lib.pb_gm_start(m, float(tol), P(hb), P(g), P(scal), st))
+        h = scal.cpu().numpy()
+        syncs += 1
+        if bnorm is None:
+            bnorm = float(np.sqrt(max(h[0], 0.0)))
+            if bnorm == 0.0:
+                x.zero_()
+                return x, {"iterations": 0, "restarts": 0, "relres": 0.0, "converged": True, "host_syncs": syncs,
+                           "cuda_graph": False}
+        relres = float(np.sqrt(max(h[1], 0.0))) / bnorm
+        if not np.isfinite(relres) or relres <= tol or it >= maxiter:
+            break
+        ck(lib.pb_gm_scale(n, P(v0), P(scal), st))
+        steps = min(m, maxiter - it)
+        k = 0
+        for j in range(steps):
+            if precond is not None:
+                ck(lib.pb_local_block_apply_dev(*precond._args(), P(precond.inv), col(j), P(z), done, st))
+                src = z.data_ptr()
+            else:
+                src = V.data_ptr() + 8 * j * n
+            a.spmv_device(src, V.data_ptr() + 8 * (j + 1) * n, st)
+            for p in range(2):
+                hp = C.c_void_p(hb.data_ptr() + 8 * p * (m + 1))
+                ww = C.c_void_p(hb.data_ptr() + 8 * (2 * (m + 1) + p))
+                ck(lib.pb_gm_dots(n, P(V), j + 1, col(j + 1), hp, P(scal), st))
+                ck(lib.pb_gm_orth(n, P(V), j + 1, hp, col(j + 1), ww, P(scal), st))
+            ck(lib.pb_gm_givens(j, m, P(H), P(hb), P(cs), P(sn), P(g), P(scal), st))
+            ck(lib.pb_gm_scale(n, col(j + 1), P(scal), st))
+            if (j + 1) % check_every == 0 or j + 1 == steps:
+                h = scal.cpu().numpy()
+                syncs += 1
+                k = int(h[6])
+                if h[5] != 0.0:
+                    break
+        it += k
+        cycles += 1
+        ck(lib.pb_gm_ysolve(m, P(H), P(g), P(y), P(scal), st))
+        if precond is not None:
+            ck(lib.pb_gm_combine(n, P(V), m, P(y), P(t), P(scal), 0, st))
+            ck(lib.pb_local_block_apply_dev(*precond._args(), P(precond.inv), P(t), P(z), None, st))
+            ck(lib.pb_gm_axpy(n, P(z), P(x), st))
+        else:
+            ck(lib.pb_gm_combine(n, P(V), m, P(y), P(x), P(scal), 1, st))
+        if k == 0:
+            break
+    return x, {"iterations": it, "restarts": max(cycles - 1, 0), "relres": relres, "converged": bool(relres <= tol),
+               "host_syncs": syncs, "cuda_graph": False}

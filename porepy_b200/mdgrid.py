@@ -192,3 +192,65 @@ def split_fractures(g: Grid, fracture_faces) -> FractureNetwork:
                                mortar_to_secondary_int=m2s, secondary_to_mortar_avg=m2s.T.tocsr(),
                                cell_volumes=np.concatenate((g.face_areas[F], g.face_areas[F]))))
     return FractureNetwork(m, fractures, interfaces, sides)
+
+
+def mortar_signs(g: Grid, mortar_to_primary) -> np.ndarray:
+    """+-1 per mortar cell: the orientation of its primary face seen from the matrix cell on that side (the face
+    normal points out of that cell: +1), as the reference's ``sign_of_mortar_sides``.  ``mortar_to_primary``: faces x
+    mortar cells, one face per mortar cell."""
+    m2p = sps.csc_matrix(mortar_to_primary)
+    m2p.eliminate_zeros()
+    if np.any(np.diff(m2p.indptr) != 1):
+        raise ValueError("every mortar cell needs exactly one primary face")
+    faces = m2p.indices
+    return np.asarray(sps.csr_matrix(g.cell_faces)[faces].sum(axis=1)).ravel().astype(float)
+
+
+def tangent_normal_basis(normal) -> np.ndarray:
+    """Rows: tangent, tangent, normal of the unit ``normal`` (3,): the first tangent is n rotated by 90 degrees in the two
+    coordinates other than n's largest one (ascending), or the unit vector of the first of them when n is aligned with an
+    axis; the second is n x t1.  The reference's ``TangentialNormalProjection`` convention."""
+    n = np.asarray(normal, float) / np.linalg.norm(normal)
+    i = int(np.argmax(np.abs(n)))
+    a, b = [q for q in range(3) if q != i]
+    t1 = np.zeros(3)
+    if np.hypot(n[a], n[b]) < 1e-8:
+        t1[a] = 1.0
+    else:
+        t1[a], t1[b] = -n[b], n[a]
+    t1 /= np.linalg.norm(t1)
+    t2 = np.cross(n, t1)
+    t2 /= np.linalg.norm(t2)
+    return np.linalg.inv(np.column_stack((t1, t2, n)))
+
+
+def fracture_local_coordinates(g: Grid, mortar_to_primary, mortar_sign, num_cells: int) -> sps.csr_matrix:
+    """3 nfc x 3 nfc rotation to the local frame of a planar fracture, the same frame in every fracture cell.  The normal
+    is the outward unit normal of the matrix cell on the mortar side of sign -1: it points from that side across the
+    fracture, so that the normal component of the jump ``sum(sign * u_j)`` (the +1 side minus the -1 side) is positive
+    when the fracture opens.  (The reference takes the side of its first mortar cell, which has sign -1 in its split
+    grids, where the original face keeps the cell it points into.)"""
+    m2p = sps.csc_matrix(mortar_to_primary)
+    m2p.eliminate_zeros()
+    sign = np.asarray(mortar_sign, float)
+    neg = np.flatnonzero(sign < 0)
+    if neg.size == 0:
+        raise ValueError("a two-sided interface needs mortar cells of sign -1")
+    f0 = int(m2p.indices[m2p.indptr[neg[0]]])
+    n = -np.asarray(g.face_normals)[:, f0] / float(np.asarray(g.face_areas)[f0])
+    return sps.kron(sps.identity(int(num_cells)), sps.csr_matrix(tangent_normal_basis(n))).tocsr()
+
+
+def fracture_contacts(net: FractureNetwork) -> list:
+    """``contact.FractureContact`` of every (planar) fracture of a network from ``split_fractures``: the projections of
+    the matching two-sided interface (one mortar cell per fracture face and side: the ``*_avg`` and ``*_int`` forms
+    coincide), the mortar signs and the local frame by the reference's conventions."""
+    from .contact import FractureContact
+    out = []
+    for fg, intf in zip(net.fractures, net.interfaces):
+        m2p = intf["mortar_to_primary_int"]
+        sign = mortar_signs(net.matrix, m2p)
+        out.append(FractureContact(m2p, m2p.T.tocsr(), intf["mortar_to_secondary_int"],
+                                   intf["secondary_to_mortar_avg"], sign, intf["cell_volumes"],
+                                   fracture_local_coordinates(net.matrix, m2p, sign, fg.num_cells)))
+    return out
