@@ -95,6 +95,11 @@ void pb_plan_destroy(pb_plan *p);
 int pb_plan_sizes(const pb_plan *p, int64_t *num_subcells, int64_t *num_subfaces,
                   int64_t *num_subhalffaces, int32_t *max_subfaces_per_node,
                   int32_t *max_subcells_per_node);
+/* The node classes the last build made (kind 0: MPFA, at plan creation; kind 1: MPSA / Biot, at pb_mpsa_upload):
+ * *count = number of classes; for the first min(count, cap) classes, the solver configuration, whether the matrix
+ * lives in the global-memory workspace, and the number of nodes.  Host only: no kernel runs. */
+int pb_plan_node_classes(const pb_plan *p, int kind, int cap, int32_t *cfg, uint8_t *a_global, int64_t *nodes,
+                         int *count);
 /* Shards: cell e of this plan is cell cells[e] of a larger (global) grid of n_source_cells cells.  The cell tensors of
  * the following pb_mpfa_upload / pb_mpsa_upload (permeability, stiffness, coupling tensors) are then the GLOBAL arrays
  * ((3,3,n_source), (9,9,n_source)) and are restricted on the device; NULL removes the map. */
@@ -377,6 +382,18 @@ int pb_gm_axpy(int64_t n, const double *z, double *x, uint64_t stream);
 
 /* time `reps` device SpMVs with CUDA events on the launching stream; returns mean ms */
 int pb_csr_spmv_bench(pb_csr *a, int reps, float *mean_ms);
+
+/* ---- diagnostics of the interaction-region solvers (solver_check.cu) ----
+ * Solver configuration cfg (0..7, the class table of plan.hpp): threads per team and the largest system order and
+ * augmented width it takes (INT_MAX for the catch-all configuration 6). */
+int pb_solver_limits(int cfg, int *team, int *max_n, int *max_w);
+/* Solve nsys dense systems with configuration cfg, one team per system, exactly as the assembly kernels run it
+ * (launch geometry, shared-memory layout, row stride (n + nrhs) | 1, rowidx starting as the identity; a_global != 0:
+ * the matrix lives in a global-memory workspace).  Host arrays: A (nsys, n, n + nrhs) row-major, the augmented
+ * [M | B]; X (nsys, n, nrhs) receives M^-1 B (NaN where the solver refused the system); ok (nsys) 1 / 0.
+ * PB_EINVAL before any launch when the system does not fit the configuration or its shared memory. */
+int pb_local_solve_batch(int cfg, int a_global, int64_t nsys, int n, int nrhs, const double *A, double *X,
+                         int32_t *ok);
 
 #ifdef __cplusplus
 }

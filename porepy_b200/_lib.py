@@ -38,6 +38,9 @@ _SIGNATURES = {
                                  _i32p, _i32p, C.POINTER(C.c_void_p)]),
     "pb_plan_destroy": (None, [C.c_void_p]),
     "pb_plan_sizes": (C.c_int, [C.c_void_p, _i64p, _i64p, _i64p, _i32p, _i32p]),
+    "pb_plan_node_classes": (C.c_int, [C.c_void_p, C.c_int, C.c_int, _i32p, _u8p, _i64p, C.POINTER(C.c_int)]),
+    "pb_solver_limits": (C.c_int, [C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int)]),
+    "pb_local_solve_batch": (C.c_int, [C.c_int, C.c_int, C.c_int64, C.c_int, C.c_int, _f64p, _f64p, _i32p]),
     "pb_plan_set_cell_map": (C.c_int, [C.c_void_p, _i64p, C.c_int64]),
     "pb_plan_set_active_nodes": (C.c_int, [C.c_void_p, _u8p]),
     "pb_plan_pattern_size": (C.c_int, [C.c_void_p, C.c_int, _i64p, _i64p]),

@@ -8,7 +8,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libporeb200.so")
-SOURCES = ["api.cu", "spmv.cu", "mpfa_launch.cu", "mpsa2d.cu", "mpsa3d.cu", "face.cu", "peaks.cu", "krylov.cu", "sparse_ops.cu", "plan_device.cu", "shard.cu", "geometry.cu", "local_blocks.cu", "gmres.cu"]
+SOURCES = ["api.cu", "spmv.cu", "mpfa_launch.cu", "mpsa2d.cu", "mpsa3d.cu", "face.cu", "peaks.cu", "krylov.cu", "sparse_ops.cu", "plan_device.cu", "shard.cu", "geometry.cu", "local_blocks.cu", "gmres.cu", "solver_check.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-O3", "-Xcompiler", "-fopenmp"]
 

@@ -490,6 +490,19 @@ extern "C" int pb_plan_sizes(const pb_plan *p, int64_t *num_subcells, int64_t *n
     return PB_OK;
 }
 
+extern "C" int pb_plan_node_classes(const pb_plan *p, int kind, int cap, int32_t *cfg, uint8_t *a_global,
+                                    int64_t *nodes, int *count) {
+    if (!p || !count || cap < 0 || (kind != 0 && kind != 1)) return fail(PB_EINVAL, "bad arguments");
+    const std::vector<NodeClass> &cls = kind == 0 ? p->mpfa_cls : p->mpsa_cls;
+    *count = (int)cls.size();
+    for (int i = 0; i < (int)cls.size() && i < cap; ++i) {
+        if (cfg) cfg[i] = cls[i].cfg;
+        if (a_global) a_global[i] = cls[i].a_global ? 1 : 0;
+        if (nodes) nodes[i] = cls[i].n;
+    }
+    return PB_OK;
+}
+
 extern "C" int pb_plan_set_active_nodes(pb_plan *p, const uint8_t *mask) {
     if (!p) return pb_fail_(PB_EINVAL, "null plan");
     if (mask) p->active.assign(mask, mask + p->H.nn); else p->active.clear();

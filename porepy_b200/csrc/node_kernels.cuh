@@ -245,6 +245,9 @@ struct RegGJ {
                 }
                 if ((key >> 8) == 0ull) { ok = false; break; }  // zero column: uniform over the team
                 const int pr = (int)(key & 0xFFull);
+                // NaN / Inf rank above every finite magnitude, so a non-finite entry in the column becomes the pivot:
+                // refuse the system as the other solvers do (the value is read from shared memory by every thread)
+                if (!isfinite(fc[pr])) { ok = false; break; }
                 const int xpiv = (ti == pr % TR) ? pr / TR : -1;
                 if (xpiv >= 0) {
                     const double inv = 1.0 / fc[pr];
@@ -397,11 +400,12 @@ struct TileGJ {
     static __device__ __forceinline__ bool try_diagonal_block(int l, const double *P0, const int *usedf,
                                                               int p0, int pw, double &iv) {
         const int mj = (l >> 2) & 3, mi = l & 3;
-        const bool bad = (mj < pw) && (usedf[p0 + mj] != 0);
-        const bool any_used = __any_sync(0xffffffffu, bad);
         const double m = (mj < pw) ? ((mi < pw) ? P0[(p0 + mj) * 4 + mi] : 0.0) : (mi == mj ? 1.0 : 0.0);
+        // a used row, or a non-finite entry (a block holding an Inf can have a finite, tame computed inverse)
+        const bool bad = ((mj < pw) && (usedf[p0 + mj] != 0)) || !isfinite(m);
+        const bool any_bad = __any_sync(0xffffffffu, bad);
         const double growth = invert_block(l, m, iv);
-        return !any_used && growth <= kGrowth;
+        return !any_bad && growth <= kGrowth;
     }
 
     template <bool TRY_FAST>
@@ -445,12 +449,15 @@ struct TileGJ {
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
             if (j < pw && !sing) {
-                // pivot choice on float-rounded magnitudes (24-bit keys, row in the low byte):
-                // one redux.sync instead of five 64-bit shuffle rounds
+                // pivot choice on the high word of |v| (sign, exponent and 20 mantissa bits; the low byte is
+                // replaced by the row): one redux.sync instead of five 64-bit shuffle rounds.  The high word is
+                // monotone over the whole double range; a float-rounded magnitude flushes everything below 1e-45
+                // to zero, which refused regular systems with graded columns.  Zero only for |v| < 2^-1034.
                 unsigned key = 0u;
 #pragma unroll
                 for (int i = 0; i < NI; ++i) {
-                    unsigned k = (__float_as_uint(fabsf((float)v[i][j])) & 0x7FFFFF00u) | (unsigned)(l + 32 * i);
+                    unsigned k = ((unsigned)(__double_as_longlong(fabs(v[i][j])) >> 32) & 0x7FFFFF00u) |
+                                 (unsigned)(l + 32 * i);
                     key = (!us[i] && k > key) ? k : key;
                 }
                 key = __reduce_max_sync(0xffffffffu, key);
@@ -476,18 +483,19 @@ struct TileGJ {
 #pragma unroll
                         for (int jj = 0; jj < 4; ++jj) prow[jj] = __shfl_sync(0xffffffffu, x[jj], ol);
                     }
-                    // fraction-free elimination: the panel copy is only used to CHOOSE the pivots
-                    // (A11^-1 is formed from the original entries below), and scaling every row by
-                    // the same pivot does not change the arg-max -> no reciprocal on the critical path
-                    const double piv = prow[j];
+                    // elimination with the multiplier f / piv.  The panel copy is only used to CHOOSE the
+                    // pivots (A11^-1 is formed from the original entries below); a fraction-free update
+                    // (v * piv - f * prow) would save the reciprocal but multiplies the copy by a pivot per
+                    // step, so a panel of columns of order s reaches s^8 after three steps and underflows
+                    const double rp = 1.0 / prow[j];
 #pragma unroll
                     for (int i = 0; i < NI; ++i) {
                         const bool me = (l == ol) && (i == os);
                         if (me) us[i] = true;
                         else {
-                            const double f = v[i][j];
+                            const double f = v[i][j] * rp;
 #pragma unroll
-                            for (int jj = j + 1; jj < 4; ++jj) v[i][jj] = v[i][jj] * piv - f * prow[jj];
+                            for (int jj = j + 1; jj < 4; ++jj) v[i][jj] -= f * prow[jj];
                         }
                     }
                 }
@@ -500,7 +508,8 @@ struct TileGJ {
             if (j == mj) prj = mypr[j];
         const double m = (prj >= 0) ? ((mi < pw) ? P0[prj * 4 + mi] : 0.0) : (mi == mj ? 1.0 : 0.0);
         const double growth = invert_block(l, m, iv);
-        if (!(growth < 1e300)) sing = true;  // inf / nan
+        // inf / nan inverse, or a non-finite pivot-block entry (1 / Inf = 0 can leave the computed inverse finite)
+        if (!(growth < 1e300) || __any_sync(0xffffffffu, !isfinite(m))) sing = true;
         if (l < 16) Ainv[l] = iv;
         if (l == 0) {
 #pragma unroll

@@ -181,6 +181,34 @@ def _lifted(plan, m, rows: np.ndarray, nc: int):
     return out
 
 
+NUM_SOLVER_CFGS = 8
+
+
+def solver_limits(cfg: int) -> tuple:
+    """``(team, max_n, max_w)`` of dense solver configuration ``cfg`` (0..7): threads per system, the largest
+    system order and the largest augmented width ``n + nrhs`` (2**31 - 1 for the catch-all configuration 6)."""
+    lib = _lib.load()
+    team, mn, mw = C.c_int(), C.c_int(), C.c_int()
+    _lib.check(lib.pb_solver_limits(int(cfg), C.byref(team), C.byref(mn), C.byref(mw)))
+    return team.value, mn.value, mw.value
+
+
+def local_solve_batch(cfg: int, A, n: int, a_global: bool = False):
+    """Solve the augmented systems ``A`` (shape (nsys, n, n + nrhs): ``[M | B]``) on the device with dense solver
+    configuration ``cfg``, exactly as the assembly kernels run it on an interaction region.  Returns ``(X, ok)``:
+    X (nsys, n, nrhs) = M^-1 B (NaN where the solver refused the system), ok (nsys,) bool."""
+    lib = _lib.load()
+    A = np.ascontiguousarray(A, dtype=np.float64)
+    if A.ndim != 3 or A.shape[1] != n or A.shape[2] <= n:
+        raise ValueError("A must have shape (nsys, n, n + nrhs) with nrhs >= 1")
+    nsys, nrhs = A.shape[0], A.shape[2] - n
+    X = np.empty((nsys, n, nrhs), np.float64)
+    ok = np.empty(nsys, np.int32)
+    _lib.check(lib.pb_local_solve_batch(int(cfg), int(bool(a_global)), nsys, int(n), int(nrhs),
+                                        _lib.ptr(A, _lib._f64p), _lib.ptr(X, _lib._f64p), _lib.ptr(ok, _lib._i32p)))
+    return X, ok.astype(bool)
+
+
 class DevicePlan:
     """Device-resident sub-cell topology + output patterns of one grid (``pb_plan``).
 
@@ -343,6 +371,21 @@ class DevicePlan:
                                           C.byref(e)))
         return dict(subcells=a.value, subfaces=b.value, subhalffaces=c.value,
                     max_subfaces_per_node=d.value, max_subcells_per_node=e.value)
+
+    def node_classes(self, kind: str) -> list:
+        """The node classes of the last build for ``kind`` ("mpfa", or "mpsa" for MPSA and Biot): a list of
+        ``(cfg, a_global, num_nodes)``, one per class, where ``cfg`` is the dense solver configuration its nodes
+        run (see ``solver_limits``) and ``a_global`` whether their matrices live in global memory."""
+        k = {"mpfa": 0, "mpsa": 1}[kind]
+        n = C.c_int()
+        _lib.check(self.lib.pb_plan_node_classes(self.h, k, 0, None, None, None, C.byref(n)))
+        cfg = np.zeros(max(n.value, 1), np.int32)
+        glob = np.zeros(max(n.value, 1), np.uint8)
+        nodes = np.zeros(max(n.value, 1), np.int64)
+        _lib.check(self.lib.pb_plan_node_classes(self.h, k, n.value, _lib.ptr(cfg, _lib._i32p),
+                                                 _lib.ptr(glob, _lib._u8p), _lib.ptr(nodes, _lib._i64p),
+                                                 C.byref(n)))
+        return [(int(cfg[i]), bool(glob[i]), int(nodes[i])) for i in range(n.value)]
 
     # ---- MPFA
     def mpfa_upload(self, perm, codes, robw, eta) -> None:
